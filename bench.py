@@ -8,6 +8,7 @@ the only collective is the weight broadcast at init.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config {2,3,4,5}] [--batch B] [--faces F] [--sampling]
     python bench.py --impl reference ...      # the CPU oracle on the host cores (bounded sample)
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's output as DIR/faces.npy
 
 --config selects a BASELINE.json configuration (index + 1): 2 = batch 1, 800 faces, greedy (default, the one the metric
 is quoted on); 3 = batch 64, 800 faces, top-k/top-p sampling; 4 = the same per GPU, meant for --gpus 8 (512 shapes);
@@ -216,6 +217,23 @@ def batched_decode_steps(arena, n_layers, B, F, sampling, contexts, steps=200, w
             "note": "decode steps only (no encoder / prefill / detokenizer); KV zero-filled, state set by ma_decode_slots_seek"}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_faces(out_dir: str, faces: torch.Tensor) -> None:
+    """Writes what MeshAnything.forward returned in the last timed step -- face coordinates [B, F, 3, 3], NaN where no
+    face was generated -- as out_dir/faces.npy in float32, so that two builds can be compared output for output.
+    Above DUMP_LIMIT_BYTES a fixed sample of whole shapes (seed 0, ascending shape index) is written instead."""
+    import numpy as np
+    a = faces.detach().float().cpu()
+    if a.numel() * 4 > DUMP_LIMIT_BYTES:
+        keep = max(1, DUMP_LIMIT_BYTES // (a[0].numel() * 4))
+        rows = torch.randperm(a.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        a = a[rows]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "faces.npy"), a.numpy())
+
+
 CONFIGS = {2: dict(batch=1, faces=800, sampling=False), 3: dict(batch=64, faces=800, sampling=True),
            4: dict(batch=64, faces=800, sampling=True), 5: dict(batch=32, faces=1600, sampling=True)}
 
@@ -237,7 +255,13 @@ def main():
     ap.add_argument("--sampling", action="store_true")
     ap.add_argument("--flags", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the output of the last timed step (rank 0's shapes) as DIR/faces.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl ours)")
     cfg = CONFIGS[args.config]
     if args.batch is None:
         args.batch = cfg["batch"]
@@ -350,9 +374,13 @@ def main():
     launches0 = capi.lib().ma_launch_count()
     sampler = ClockSampler(local)
     sampler.start()
-    ms, out = timed(one_step_resident, args.steps)
-    clocks = sampler.stop()
+    try:
+        ms, out = timed(one_step_resident, args.steps)
+    finally:
+        clocks = sampler.stop()   # never leave the nvidia-smi sampler running
     launches = capi.lib().ma_launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_faces(args.dump_outputs, out)
     ms_e2e, out_e2e = timed(one_step_e2e, args.steps)
     e2e_remeasured = None
     if ms_e2e > 1.5 * ms:   # the e2e pass only adds ~50 KB of copies: a large gap is a disturbed measurement, not the path
