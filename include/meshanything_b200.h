@@ -279,6 +279,26 @@ size_t ma_sample_surface_workspace_bytes(int n_faces);
 int ma_sample_surface(const float* vertices, const int32_t* faces, int n_faces, int n_samples, unsigned long long seed,
                       void* out_pc_normal, int32_t* out_face_idx, void* ws, void* stream);
 
+/* ---- watertight remesh (`--mc`): unsigned distance field + marching cubes -------------------------------------
+ * Grid of size^3 nodes (size in 32..256; the reference uses 2^7), spacing h = 2 / size, node (i, j, k) at
+ * (-1 + i h, -1 + j h, -1 + k h); fields are fp32 [size][size][size] indexed [i][j][k], k fastest.
+ *
+ * ma_mesh_udf: vertices fp32 [V][3] (normalised to +-0.9), faces int32 [F][3] (indices in [0, V), not checked here) ->
+ * out_field[n] = min(d(n), 2h), d the exact distance from node n to the nearest triangle; zero-area triangles count by
+ * their edges and points.  Bit-identical for any order of the faces.  Needs no workspace. */
+int ma_mesh_udf(const float* vertices, const int32_t* faces, int n_faces, int size, float* out_field, void* stream);
+
+/* Marching cubes of `field` at `level` (inside: field < level), one vertex per crossing grid edge, triangles oriented
+ * with (v1 - v0) x (v2 - v0) towards increasing field; closed wherever the level set stays inside the grid.
+ * ma_marching_cubes_count writes out_counts (device int32 [2]) = (vertices, triangles) and the per-node offsets into ws
+ * (ma_marching_cubes_workspace_bytes(size) bytes); ma_marching_cubes_emit, given the same field, level and ws, writes
+ * out_vertices fp32 [V][3] = ((index * h) - 1) * inv_scale + (cx, cy, cz) and out_faces int32 [F][3], vertices in
+ * order of owning node then axis, triangles in cell order then table order. */
+size_t ma_marching_cubes_workspace_bytes(int size);
+int ma_marching_cubes_count(const float* field, int size, float level, int32_t* out_counts, void* ws, void* stream);
+int ma_marching_cubes_emit(const float* field, int size, float level, float inv_scale, float cx, float cy, float cz,
+                           float* out_vertices, int32_t* out_faces, void* ws, void* stream);
+
 /* number of kernels launched by the library since load (bench.py's gpu_launches) */
 unsigned long long ma_launch_count(void);
 

@@ -1,9 +1,11 @@
 """Drop-in for /root/reference/mesh_to_pc.py: mesh -> (4096, 6) fp16 point cloud with normals.
 
-Uses trimesh / mesh2sdf / skimage when they are installed (same calls as the reference); otherwise a
-small numpy implementation of area-weighted surface sampling (what `trimesh.Trimesh.sample` does) is
-used (OBJ and ASCII/binary PLY readers included) and `marching_cubes=True` raises (mesh2sdf is required for the
-watertight conversion).
+With a CUDA device the whole path runs in CUDA: `marching_cubes=True` (`--mc`) rebuilds the mesh as a watertight double shell
+(distance field + marching cubes, csrc/watertight.cu) and the points are drawn by the CUDA surface sampler.  Without a
+GPU, or with MA_PC_SAMPLER=host, it uses trimesh / mesh2sdf / skimage when they are installed (same calls as the
+reference); otherwise a small numpy implementation of area-weighted surface sampling (what `trimesh.Trimesh.sample`
+does) is used (OBJ and ASCII/binary PLY readers included) and `marching_cubes=True` raises (mesh2sdf is required for the
+host watertight conversion).
 """
 import numpy as np
 
@@ -146,9 +148,39 @@ def normalize_vertices(vertices, scale=0.9):
     return (vertices - centre) * factor, centre, factor
 
 
+def _watertight_gpu(gpu, mesh, octree_depth):
+    """(vertices fp32 [V, 3], faces int32 [F, 3]) of the watertight remesh, on the device: the mesh normalised to +-0.9
+    on the host in float64, min(distance, 2h) on the 2^depth grid (ma_mesh_udf), marching cubes at level h = 2/size
+    mapped back to the input frame (ma_marching_cubes_*)."""
+    capi, torch = gpu
+    if not 5 <= octree_depth <= 8:
+        raise ValueError(f"octree_depth must be in 5..8, got {octree_depth}")
+    vertices = np.asarray(mesh.vertices, dtype=np.float64)
+    faces = np.asarray(mesh.faces, dtype=np.int64)
+    if vertices.ndim != 2 or vertices.shape[1] != 3 or faces.ndim != 2 or faces.shape[1] != 3 or len(faces) == 0:
+        raise ValueError(f"watertight remesh needs vertices [V, 3] and at least one face [F, 3], got "
+                         f"{vertices.shape} / {faces.shape}")
+    if not np.isfinite(vertices).all():
+        raise ValueError("watertight remesh: the mesh has non-finite vertices")
+    if faces.min() < 0 or faces.max() >= len(vertices):
+        raise ValueError(f"watertight remesh: face indices outside [0, {len(vertices)})")
+    size = 2 ** octree_depth
+    unit_vertices, centre, factor = normalize_vertices(vertices)
+    dev = torch.device("cuda", torch.cuda.current_device())
+    v = torch.as_tensor(unit_vertices.astype(np.float32), device=dev)
+    f = torch.as_tensor(faces.astype(np.int32), device=dev)
+    field = capi.mesh_udf(v, f, size)
+    return capi.marching_cubes(field, 2 / size, inv_scale=1.0 / factor, centre=centre)
+
+
 def export_to_watertight(normalized_mesh, octree_depth: int = 7):
-    """Watertight remesh used by `--mc` (reference mesh_to_pc.py:13-40): unsigned distance field on a 2^depth grid
-    (mesh2sdf), marching cubes at iso level 2/size, mapped back to the input frame."""
+    """Watertight remesh used by `--mc` (reference mesh_to_pc.py:13-40): unsigned distance field on a 2^depth grid,
+    marching cubes at iso level 2/size, mapped back to the input frame.  With a CUDA device it runs in CUDA and returns a
+    SimpleMesh; otherwise it needs mesh2sdf / skimage / trimesh, as the reference does."""
+    gpu = _gpu_sampler()
+    if gpu is not None:
+        v, f = _watertight_gpu(gpu, normalized_mesh, octree_depth)
+        return SimpleMesh(v.cpu().numpy(), f.cpu().numpy())
     try:
         import mesh2sdf.core
         import skimage.measure
@@ -181,18 +213,24 @@ def _gpu_sampler():
 
 def process_mesh_to_pc(mesh_list, marching_cubes=False, sample_num=4096):
     """[mesh] -> ([fp16 (sample_num, 6) points + face normals], [mesh actually sampled]).  On a GPU box the points are
-    drawn by the CUDA sampler (seeded from numpy's generator, so `set_seed` still decides them)."""
+    drawn by the CUDA sampler (seeded from numpy's generator, so `set_seed` still decides them), and with
+    `marching_cubes=True` the watertight remesh (a SimpleMesh in `used`) is built in CUDA too."""
     clouds, used = [], []
     gpu = _gpu_sampler()
     for mesh in mesh_list:
-        if marching_cubes:
+        if marching_cubes and gpu is not None:        # the rebuilt mesh stays on the device for the sampler
+            v, f = _watertight_gpu(gpu, mesh, 7)
+            mesh = SimpleMesh(v.cpu().numpy(), f.cpu().numpy())
+            print("MC over!")
+        elif marching_cubes:
             mesh = export_to_watertight(mesh)
             print("MC over!")
         if gpu is not None:
             capi, torch = gpu
             dev = torch.device("cuda", torch.cuda.current_device())
-            v = torch.as_tensor(np.asarray(mesh.vertices, dtype=np.float32), device=dev)
-            f = torch.as_tensor(np.asarray(mesh.faces, dtype=np.int32), device=dev)
+            if not marching_cubes:
+                v = torch.as_tensor(np.asarray(mesh.vertices, dtype=np.float32), device=dev)
+                f = torch.as_tensor(np.asarray(mesh.faces, dtype=np.int32), device=dev)
             seed = int(np.random.randint(0, 2 ** 31 - 1))
             clouds.append(capi.sample_surface(v, f, sample_num, seed=seed).cpu().numpy())
             used.append(mesh)

@@ -14,7 +14,7 @@ LIB_DIR = os.path.join(HERE, "lib")
 # travel to the GPU box side by side); the default uses the mixed-precision FMA (SASS FHFMA), see canon.cuh
 VARIANT = "_nofhfma" if os.environ.get("MA_B200_NO_FHFMA") == "1" else ""
 LIB = os.path.join(LIB_DIR, f"libmeshanything_b200{VARIANT}.so")
-SOURCES = ["gemm_canon.cu", "attention.cu", "attention_stream.cu", "elementwise.cu", "decode_fast.cu", "decode_mega.cu", "api.cu", "glue.cu", "gemm_tc.cu", "gemm_ws.cu", "attention_tc.cu", "api_encoder.cu", "surface.cu"]
+SOURCES = ["gemm_canon.cu", "attention.cu", "attention_stream.cu", "elementwise.cu", "decode_fast.cu", "decode_mega.cu", "api.cu", "glue.cu", "gemm_tc.cu", "gemm_ws.cu", "attention_tc.cu", "api_encoder.cu", "surface.cu", "watertight.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 if VARIANT:

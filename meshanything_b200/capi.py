@@ -45,6 +45,7 @@ EXPORTS = [
     "ma_decode_slots_init", "ma_decode_slot_prefill", "ma_decode_slots_step", "ma_decode_slots_poll",
     "ma_mega_set_debug", "ma_linear_ws_set_mode", "ma_decode_slots_seek", "ma_decode_slot_stream", "ma_linear_ws_scratch_bytes", "ma_linear_ws_f16",
     "ma_sample_surface_workspace_bytes", "ma_sample_surface", "ma_tensor_core_linear_counts",
+    "ma_mesh_udf", "ma_marching_cubes_workspace_bytes", "ma_marching_cubes_count", "ma_marching_cubes_emit",
 ]
 
 
@@ -111,6 +112,12 @@ def lib():
     L.ma_sample_surface_workspace_bytes.argtypes = [C.c_int]
     L.ma_sample_surface_workspace_bytes.restype = C.c_size_t
     L.ma_sample_surface.argtypes = [_vp, _vp, C.c_int, C.c_int, C.c_ulonglong, _vp, _vp, _vp, _vp]
+    L.ma_mesh_udf.argtypes = [_vp, _vp, C.c_int, C.c_int, _vp, _vp]
+    L.ma_marching_cubes_workspace_bytes.argtypes = [C.c_int]
+    L.ma_marching_cubes_workspace_bytes.restype = C.c_size_t
+    L.ma_marching_cubes_count.argtypes = [_vp, C.c_int, C.c_float, _vp, _vp, _vp]
+    L.ma_marching_cubes_emit.argtypes = [_vp, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, _vp, _vp,
+                                         _vp, _vp]
     L.ma_linear_tc_f16.argtypes = [_vp, _vp, _vp, C.c_int, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _vp]
     L.ma_set_tensor_cores.argtypes = [C.c_int]
     L.ma_tensor_core_linear_counts.argtypes = [C.POINTER(C.c_ulonglong), C.POINTER(C.c_ulonglong)]
@@ -170,6 +177,40 @@ def sample_surface(vertices: torch.Tensor, faces: torch.Tensor, n_samples: int, 
     check(lib().ma_sample_surface(ptr(v), ptr(f), F, n_samples, int(seed), ptr(out), ptr(idx), ptr(ws), stream_ptr()),
           "ma_sample_surface")
     return (out, idx) if want_index else out
+
+
+def mesh_udf(vertices: torch.Tensor, faces: torch.Tensor, size: int) -> torch.Tensor:
+    """Unsigned distance field min(d, 2h) of a mesh normalised to +-0.9 on the size^3 grid of [-1, 1 - h]^3, h = 2/size:
+    fp32 [size, size, size] indexed [i][j][k].  Face indices must lie in [0, V) (the caller checks)."""
+    _need_cuda(vertices, faces)
+    v = vertices.to(torch.float32).contiguous()
+    f = faces.to(torch.int32).contiguous()
+    field = torch.empty((size, size, size), dtype=torch.float32, device=v.device)
+    check(lib().ma_mesh_udf(ptr(v), ptr(f), f.shape[0], size, ptr(field), stream_ptr()), "ma_mesh_udf")
+    return field
+
+
+def marching_cubes(field: torch.Tensor, level: float, inv_scale: float = 1.0, centre=(0.0, 0.0, 0.0)):
+    """Closed, outward-oriented level set of a cubic fp32 field -> (vertices fp32 [V, 3], faces int32 [F, 3]) on the
+    device; vertex = ((grid index * h) - 1) * inv_scale + centre.  Reads the two counts back (one synchronisation)."""
+    _need_cuda(field)
+    size = field.shape[0]
+    if field.dim() != 3 or field.shape != (size, size, size):
+        raise ValueError(f"marching_cubes: field must be a cube, got {tuple(field.shape)}")
+    fd = field.to(torch.float32).contiguous()
+    ws = torch.empty(max(lib().ma_marching_cubes_workspace_bytes(size), 1), dtype=torch.uint8, device=fd.device)
+    counts = torch.empty(2, dtype=torch.int32, device=fd.device)
+    check(lib().ma_marching_cubes_count(ptr(fd), size, C.c_float(level), ptr(counts), ptr(ws), stream_ptr()),
+          "ma_marching_cubes_count")
+    nv, nf = counts.tolist()
+    verts = torch.empty((nv, 3), dtype=torch.float32, device=fd.device)
+    faces = torch.empty((nf, 3), dtype=torch.int32, device=fd.device)
+    if nf > 0:
+        cx, cy, cz = (float(c) for c in centre)
+        check(lib().ma_marching_cubes_emit(ptr(fd), size, C.c_float(level), C.c_float(inv_scale), C.c_float(cx),
+                                           C.c_float(cy), C.c_float(cz), ptr(verts), ptr(faces), ptr(ws), stream_ptr()),
+              "ma_marching_cubes_emit")
+    return verts, faces
 
 
 def tensor_core_linear_counts():
